@@ -2,6 +2,7 @@
 """bench.py -- throughput of the 3D-GCN hot path (BASELINE.json metric: 3D-GCN fwd point clouds/sec @1028 pts).
 
   python bench.py --gpus N --steps K --warmup W            # our arm (CUDA path)
+  python bench.py ... --dump-outputs DIR                   # + the last timed step's outputs as DIR/<name>.npy
   python bench.py --impl reference --gpus N --steps K ...  # CPU arm: the UNMODIFIED reference modules (oracle/_ref/pyref,
                                                            # staged from /root/reference by build()) on host cores;
                                                            # the oracle port only when that staging is absent
@@ -348,12 +349,15 @@ def run_ours(args):
     for i in range(args.steps):
         flush.zero_()
         ev[i][0].record()
-        step(*dev_sets[i % n_sets])
+        out = step(*dev_sets[i % n_sets])
         ev[i][1].record()
     barrier()
     wall = time.perf_counter() - wall0
     launches = launches_per_step * args.steps
     dev_ms = sum(a.elapsed_time(b) for a, b in ev)
+    if args.dump_outputs and rank == 0:
+        # the graph's static outputs are overwritten by the later loops: copy the last timed step's now
+        dump_outputs(args.dump_outputs, out)
 
     # ---- encoder only (SURVEY 8d: "report encoder-only clouds/s -- the optimisation target -- and full-network clouds/s
     # separately"): Face_Enc.forward alone, same clouds (centred like PoseNet9D.py:48), same replay/flush/event protocol
@@ -459,6 +463,26 @@ def run_ours(args):
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_CAP_BYTES = 64 << 20
+
+
+def dump_outputs(directory, out):
+    """Write the outputs of one forward (the dict a caller of PoseNet9D receives) as DIR/<name>.npy, float32.
+    The inputs and weights are seeded, so two builds run with the same arguments can be compared file for file.
+    All files together stay within DUMP_CAP_BYTES: an array larger than its share keeps a fixed, seeded sample of its
+    rows (the same rows in every run)."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    share = DUMP_CAP_BYTES // max(len(out), 1)
+    for name, t in out.items():
+        a = t.detach().float().cpu().numpy()
+        if a.nbytes > share:
+            a = a.reshape(a.shape[0], -1) if a.ndim > 1 and a[0].nbytes <= share else a.reshape(-1, 1)
+            keep = share // a[0].nbytes
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+        np.save(os.path.join(directory, f"{name}.npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------ secondary records
@@ -877,7 +901,13 @@ def main():
     ap.add_argument("--train-batch", type=int, default=256, help="global batch of the training step")
     ap.add_argument("--optimizer", default="ranger", choices=["ranger", "adam"],
                     help="--mode train: the reference's Ranger (fused kernels) or torch's fused Adam")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (inference arm, rank 0)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.mode != "infer"):
+        ap.error("--dump-outputs applies to the inference arm (--impl ours --mode infer)")
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

@@ -14,7 +14,8 @@ ROOT = os.path.dirname(HERE)
 
 def test_reference_face_enc_runs_unchanged_on_our_gcn3d():
     if not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "pyref", "network", "fs_net_repo", "FaceRecon.py")):
-        pytest.skip("oracle/_ref/pyref not staged (no /root/reference at build time)")
+        pytest.skip("needs the original project's FaceRecon.py, staged into oracle/_ref/pyref by build() from the "
+                    "unmodified reference sources, which this repository does not ship")
     # a fresh interpreter: the module swap must happen before the reference's FaceRecon is imported
     p = subprocess.run([sys.executable, os.path.join(HERE, "dropin_face_enc.py")], capture_output=True, text=True, timeout=600)
     assert p.returncode == 0, p.stderr[-3000:]

@@ -46,7 +46,8 @@ def test_gemm_args_struct_layout_matches_header():
 
 
 def test_no_cpu_fallback():
-    from tgpose_b200 import gcn3d
+    from tgpose_b200 import _lib, gcn3d
+    n0 = _lib.launch_count()
     x = torch.rand(1, 16, 3)
     with pytest.raises(RuntimeError):
         gcn3d.get_neighbor_index(x, 4)
@@ -66,6 +67,8 @@ def test_no_cpu_fallback():
         with pytest.raises(RuntimeError):
             head.train()(torch.rand(2, posenet.FEAT_C, 32))
     del dec
+    # every refusal happens before a launch: a kernel handed host addresses faults the CUDA context after the call returned
+    assert _lib.launch_count() == n0
 
 
 def test_state_dict_names_and_shapes():

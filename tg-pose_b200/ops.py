@@ -41,8 +41,16 @@ def _run(name, cfn, *args):
     _lib.check(rc, "tgp_" + name)
 
 
+def _ptr(t):
+    """device address of a tensor handed to the C-ABI.  A host tensor is refused here, before anything is launched: a
+    kernel given a host address faults the whole CUDA context, asynchronously, long after the call returned."""
+    if not t.is_cuda:
+        raise RuntimeError("expected a CUDA tensor (tg-pose_b200 has no CPU path)")
+    return t.data_ptr()
+
+
 def _p(t):
-    return ctypes.c_void_p(t.data_ptr()) if t is not None else None
+    return ctypes.c_void_p(_ptr(t)) if t is not None else None
 
 
 def _stream():
@@ -186,7 +194,7 @@ def concat_rows(sources, B, N, want_raw=True, want_split=False, mixed=False):
         if idx is not None:
             idx = idx.to(torch.int32).contiguous()
             keep.append(idx)
-        arr[i] = _lib.ConcatSrc(t.data_ptr(), t.shape[1], t.stride(0), idx.data_ptr() if idx is not None else None, n_src)
+        arr[i] = _lib.ConcatSrc(_ptr(t), t.shape[1], t.stride(0), _ptr(idx) if idx is not None else None, n_src)
         total += t.shape[1]
     M = B * N
     raw = torch.empty((M, total), dtype=torch.float32, device=dev) if want_raw else None
@@ -314,35 +322,35 @@ def gemm(A, Bmat, b_is_nk, segs, bias=None, group_bias=None, rows_per_group=0, r
         A_split = B_split = None
     a = GemmArgs()
     if A is not None:
-        a.A, a.lda = A.data_ptr(), A.stride(0)
-    a.Bmat, a.ldb, a.b_is_nk = Bmat.data_ptr(), Bmat.stride(0), 1 if b_is_nk else 0
+        a.A, a.lda = _ptr(A), A.stride(0)
+    a.Bmat, a.ldb, a.b_is_nk = _ptr(Bmat), Bmat.stride(0), 1 if b_is_nk else 0
     if A_split is not None and B_split is not None:
-        a.A_split, a.B_split = A_split.data_ptr(), B_split.data_ptr()
+        a.A_split, a.B_split = _ptr(A_split), _ptr(B_split)
     a.mixed = int(mixed)          # 0: 3xTF32 operands, 1: mixed, 2: mixed with a w16 weight operand (third pass fp16(a).lo16(b))
     a.a_kp, a.a_group_cols = int(a_kp), int(a_group_cols)      # block-diagonal contraction (tgp_gemm_args.a_group_cols)
     if mixed:
         assert A_split is not None and B_split is not None, "mixed operands must be supplied (split_mixed / mode-4 epilogue)"
     a.M, a.K, a.Ncols = M, K, Ncols
-    a.bias = bias.data_ptr() if bias is not None else None
-    a.group_bias = group_bias.data_ptr() if group_bias is not None else None
+    a.bias = _ptr(bias) if bias is not None else None
+    a.group_bias = _ptr(group_bias) if group_bias is not None else None
     a.rows_per_group = rows_per_group
     if res1 is not None:
         assert res1.stride(-1) == 1
-        a.res1, a.ld_res1 = res1.data_ptr(), res1.stride(0)
+        a.res1, a.ld_res1 = _ptr(res1), res1.stride(0)
     if res2 is not None:
         assert res2.stride(-1) == 1
-        a.res2, a.ld_res2 = res2.data_ptr(), res2.stride(0)
+        a.res2, a.ld_res2 = _ptr(res2), res2.stride(0)
     for nm, ix, rs_ in (("res1_idx", res1_idx, res1), ("res2_idx", res2_idx, res2)):
         if ix is not None:      # gathered residual: output row m adds row ix[m] of the residual matrix
             assert rs_ is not None and ix.dtype == torch.int32 and ix.is_contiguous() and ix.numel() == M
-            setattr(a, nm, ix.data_ptr())
-    a.scale = scale.data_ptr() if scale is not None else None
-    a.shift = shift.data_ptr() if shift is not None else None
+            setattr(a, nm, _ptr(ix))
+    a.scale = _ptr(scale) if scale is not None else None
+    a.shift = _ptr(shift) if shift is not None else None
     a.relu = 1 if relu else 0
-    a.neg_slope = neg_slope.data_ptr() if neg_slope is not None else None
+    a.neg_slope = _ptr(neg_slope) if neg_slope is not None else None
     a.nseg = len(segs)
     for i, (c0, c1, t, mode, sw) in enumerate(segs):
-        a.seg[i] = OutSeg(c0, c1, mode, sw, t.stride(0) if mode in (0, 2, 4, 5) else 0, t.data_ptr())
+        a.seg[i] = OutSeg(c0, c1, mode, sw, t.stride(0) if mode in (0, 2, 4, 5) else 0, _ptr(t))
     name = "gemm_tc" if A_split is not None and B_split is not None else "gemm"
     if EVENT_LOG is not None:
         # algo_flops: flops of the REFERENCE's contraction this launch stands for, when the launch is a factored piece of it
